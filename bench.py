@@ -275,6 +275,19 @@ def first_stream_divergence(a, b):
     return None if len(a) == len(b) else {"window": min(len(a), len(b)), "token": 0, "resident": None, "e2e": None}
 
 
+def dump_outputs(out_dir: str, streams, pos, suffix: str = "") -> None:
+    """What one step of the resident path returns, as .npy files: tokens (songs, windows, new tokens) float64 generated ids (-1
+    pads a window that stopped early) and, with the DiT stage, positions (songs, 2, points) float32 osu! pixels."""
+    os.makedirs(out_dir, exist_ok=True)
+    tokens = np.full((len(streams), len(streams[0]), max(len(w) for st in streams for w in st)), -1.0)
+    for k, st in enumerate(streams):
+        for i, w in enumerate(st):
+            tokens[k, i, :len(w)] = w
+    np.save(os.path.join(out_dir, f"tokens{suffix}.npy"), tokens)
+    if pos is not None:
+        np.save(os.path.join(out_dir, f"positions{suffix}.npy"), torch.stack(pos).float().cpu().numpy())
+
+
 def main() -> None:
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -296,6 +309,9 @@ def main() -> None:
     ap.add_argument("--mega", type=int, default=2, help="2 = dataflow token-loop megakernel (default), 1 = grid-barrier megakernel, 0 = CUDA-graph replay per token")
     ap.add_argument("--cpu-threads", type=int, default=int(os.environ.get("MB200_CPU_THREADS", "0")),
                     help="torch threads of the CPU arm (0 = min(cores, 16): measured best on the GPU box; 32+ threads slow a batch-1 decoder down)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="--impl b200: write the token ids and DiT positions of the last timed step to DIR/tokens.npy, "
+                         "DIR/positions.npy (with several ranks: tokens_rank<r>.npy, ...) to compare two builds output for output")
     args = ap.parse_args()
     rank, world, local = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("LOCAL_RANK", 0))
     if args.impl == "reference":
@@ -432,6 +448,8 @@ def main() -> None:
     with ClockSampler(local) as clk:
         ms, toks, launches, streams, pos = timed(step_resident, args.steps, args.warmup)
     clocks = clk.summary()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, streams, pos, f"_rank{rank}" if world > 1 else "")
     for ev in step_resident.events:
         stage_ms["encode"] += ev[0].elapsed_time(ev[1]); stage_ms["decode"] += ev[1].elapsed_time(ev[2]); stage_ms["dit"] += ev[2].elapsed_time(ev[3])
     n_ev = max(1, len(step_resident.events))

@@ -126,3 +126,66 @@ def dit_chunk_case(dc, T: int = 300, seed: int = 8):
 def dit_chunk_noise(k: int, shape, steps: int = 100) -> torch.Tensor:
     g = torch.Generator().manual_seed(1000 + k)
     return torch.randn(steps, *shape, generator=g)
+
+
+PIN_LOGIT_STRIDE = 7      # every 7th vocabulary column of the v29 logits is stored (524 of 3667), beside the full-row argmax
+
+
+def v29_logits_case(cfg):
+    """One window of PCM and 12 decoder ids for a teacher-forced pass at v29 dimensions."""
+    g = torch.Generator().manual_seed(0)
+    pcm = torch.randn(1, cfg.samples_per_window, generator=g) * 0.1
+    ids = torch.randint(17, cfg.vocab_size_in, (1, 12), generator=g)
+    return pcm, ids
+
+
+def context_embedding_case(T: int = 37):
+    """Object times (ms), distances (px) and types of the seq_c layout (diffusion_pipeline.py:380-387)."""
+    g = torch.Generator().manual_seed(4)
+    seq_o = torch.rand(T, generator=g) * 180000.0
+    seq_d = torch.rand(T, generator=g) * 400.0
+    types = torch.randint(0, 16, (T,), generator=g)
+    return seq_o, seq_d, types
+
+
+def bench_window_case(cfg):
+    """The bench workload's second window with 10 new tokens: (model_kwargs, generate_kwargs, prompt length)."""
+    import bench
+    g = torch.Generator().manual_seed(0)
+    pcm = torch.randn(1, cfg.samples_per_window, generator=g) * 0.1
+    prompt = torch.tensor([bench.prompt_for(1, [list(range(100, 164))])])
+    P = prompt.shape[1]
+    gk = bench.gen_kwargs(1, 211, P)
+    gk.update(max_length=P + 10, min_new_tokens=10, precision="fp32")
+    return dict(inputs=pcm, decoder_input_ids=prompt, decoder_attention_mask=prompt.ne(0)), gk, P
+
+
+def slider_class_cases():
+    """(curve type, control points, length) of 60 seeded sliders per curve type, some Bezier / Catmull ones with a red anchor."""
+    import numpy as np
+    rng = np.random.default_rng(7)
+    out = []
+    for typ in ("Bezier", "PerfectCurve", "Catmull", "Linear"):
+        for k in range(60):
+            ncp = int(rng.integers(2, 10)) if typ != "PerfectCurve" else int(rng.choice([3, 3, 4, 2]))
+            cps = (rng.random((ncp, 2)) * np.array([512, 384])).astype(np.float32)
+            if ncp >= 4 and k % 4 == 0:
+                j = int(rng.integers(1, ncp - 2)); cps[j + 1] = cps[j]
+            out.append((typ, cps, float(rng.random() * 500 + 5)))
+    return out
+
+
+def trim_cases(layout):
+    """(tokens, trim_lookback, trim_lookahead) cases around both zones; v29 window = 8184 ms, lookback 0.5, lookahead 0.4."""
+    ts, te, circle = layout.time_shift_start, layout.time_shift_end, layout.event_start["circle"]
+    eos, ceos = layout.eos_id, layout.context_eos["map"]
+    lb_end, la_begin = layout.lookback_end(4092.0), layout.lookback_end(4910.4)
+    body = [circle, ts + 500, circle, ts + 520]
+    out = []
+    for tail in ([], [eos], [ceos], [ceos, eos], [eos, eos, ceos]):
+        for last in (ts, lb_end - 1, lb_end, la_begin - 1, la_begin, te - 1, circle):
+            for tlb in (False, True):
+                for tla in (False, True):
+                    out.append((body + [circle, last] + tail, tlb, tla))
+    out += [([], True, True), ([eos], True, True), ([ts + 3], True, True), ([te - 1, eos], False, True)]
+    return out

@@ -1,4 +1,5 @@
-"""Generate tests/golden/*.npz from the UNMODIFIED reference classes (run in the build container: needs /root/reference).
+"""Generate tests/golden/*.npz from the UNMODIFIED reference classes (needs a checkout of the reference project, located by
+oracle/ref_import.py).  The tests only read the stored outputs.
 
 TEST INFRASTRUCTURE.  Usage:  python -m oracle.make_golden
 Inputs are regenerated from seeds by the tests (torch CPU generator); only reference OUTPUTS are stored.
@@ -153,6 +154,7 @@ def main():
                                     np.log(diff.betas), diff.posterior_mean_coef1, diff.posterior_mean_coef2], 1)
     np.savez_compressed(os.path.join(OUT, "dit_reference.npz"), **dit_out, **{f"meta_{k}": v for k, v in meta.items()})
     make_slider_golden(meta)
+    make_pins_golden(meta)
     for f in sorted(os.listdir(OUT)):
         print(f, os.path.getsize(os.path.join(OUT, f)))
 
@@ -184,6 +186,72 @@ def make_slider_golden(meta=None):
     np.savez_compressed(os.path.join(OUT, "slider_reference.npz"), types=np.array(types, dtype=np.int32), offsets=np.array(offs, dtype=np.int32),
                         points=np.concatenate(pts).astype(np.float32), lengths=np.array(lens, dtype=np.float32), max_length=np.array(maxl),
                         end_pos=np.stack(ends), **({f"meta_{k}": v for k, v in (meta or {}).items()}))
+
+
+def make_pins_golden(meta=None):
+    """Outputs of single reference functions at v29 dimensions or on host-side helpers (tests/golden/reference_pins.npz):
+    `Mapperatorinator.forward` logits, `server.model_generate` ids on the bench's second window, `timestep_embedding`,
+    `SliderPath` end points and the token-level result of `Processor.add_predicted_tokens_to_context`."""
+    import dataclasses
+    import types as _types
+    from mapperatorinator_b200 import v29_model_config
+    from oracle import ref_import
+    torch.set_grad_enabled(False)
+    out = {}
+    # ---- teacher-forced logits and greedy ids of the bench's second window, whisper-small dimensions ----
+    cfg = dataclasses.replace(v29_model_config(), mel=MelConfig("torchaudio", n_mels=80))
+    model, tok, _ = ref_build.reference_model(cfg, mel_impl="torchaudio")
+    assert TokenLayout.from_tokenizer(tok) == TokenLayout.from_json(os.path.join(ROOT, "tests", "golden", "tokenizer_v29.json"))
+    ref_build.load_state_dict_into_reference(model, init_model_state_dict(cfg, 0))
+    pcm, ids = cases.v29_logits_case(cfg)
+    logits = model(frames=pcm, decoder_input_ids=ids, decoder_attention_mask=ids.ne(0)).logits.float()
+    out["v29_logits_sample"] = logits.numpy()[:, :, ::cases.PIN_LOGIT_STRIDE]
+    out["v29_logits_argmax"] = logits.argmax(-1).numpy()
+    from osuT5.osuT5.inference.server import model_generate
+    mk, gk, _ = cases.bench_window_case(cfg)
+    out["bench_window_ids"] = model_generate(model, tok, mk, gk)[0].numpy()
+    del model
+    # ---- timestep_embedding of the seq_c layout ----
+    from osu_diffusion import timestep_embedding
+    seq_o, seq_d, _ = cases.context_embedding_case()
+    out["timestep_embedding_time"] = timestep_embedding(seq_o * 0.1, 128).numpy()
+    out["timestep_embedding_distance"] = timestep_embedding(seq_d, 128).numpy()
+    # ---- SliderPath end points (max_length 0 marks a degenerate path the test skips) ----
+    SP = ref_import.reference_slider_path()
+    mls, ends = [], []
+    for typ, cps, length in cases.slider_class_cases():
+        sp = SP(typ, cps)
+        ml = float(sp.get_distance())
+        mls.append(ml)
+        ends.append(np.asarray(sp.position_at(length / ml), dtype=np.float64) if ml != 0 else np.zeros(2))
+    out["slider_class_max_length"] = np.array(mls)
+    out["slider_class_end_pos"] = np.stack(ends)
+    # ---- the tokens add_predicted_tokens_to_context hands to _decode, on a stand-in `self` (processor.py:1022-1052) ----
+    from osuT5.osuT5.inference import processor as rp
+    from osuT5.osuT5.tokenizer import ContextType
+    layout = TokenLayout.from_json(os.path.join(ROOT, "tests", "golden", "tokenizer_v29.json"))
+    seen, trimmed = [], []
+    fake = _types.SimpleNamespace(
+        tokenizer=_types.SimpleNamespace(eos_id=layout.eos_id, context_eos={ContextType(k): v for k, v in layout.context_eos.items()}),
+        lookback_time_range=range(layout.time_shift_start, layout.lookback_end(4092.0)),                 # processor.py:85
+        lookahead_time_range=range(layout.lookback_end(4910.4), layout.time_shift_end),                  # processor.py:88
+        types_first=True, eos_time=0.0, lookahead_max_time=4910.4,
+        _decode=lambda toks, frame_time: seen.append(list(toks)) or [], _trim_events_after_time=lambda *a: None)
+    old = rp.update_event_times
+    rp.update_event_times = lambda *a, **k: None
+    try:
+        for types_first in (True, False):
+            fake.types_first = types_first
+            for toks, tlb, tla in cases.trim_cases(layout):
+                seen.clear()
+                ctx = {"context_type": ContextType("map"), "events": [], "event_times": []}
+                rp.Processor.add_predicted_tokens_to_context(fake, ctx, torch.tensor(toks, dtype=torch.long).tolist(), 1234.0, tlb, tla)
+                trimmed.append(seen[0])
+    finally:
+        rp.update_event_times = old
+    out["trim_offsets"] = np.cumsum([0] + [len(s) for s in trimmed])          # types_first=True cases, then types_first=False
+    out["trim_tokens"] = np.array(sum(trimmed, []), dtype=np.int64)
+    np.savez_compressed(os.path.join(OUT, "reference_pins.npz"), **out, **({f"meta_{k}": v for k, v in (meta or {}).items()}))
 
 
 if __name__ == "__main__":

@@ -1,6 +1,6 @@
-"""Build the UNMODIFIED reference models (build container only; needs /root/reference).
+"""Build the UNMODIFIED reference models (needs a checkout of the reference project, see oracle/ref_import.py).
 
-TEST INFRASTRUCTURE.  Used by oracle/make_golden.py and tests/test_oracle_vs_reference.py to pin the oracle.
+TEST INFRASTRUCTURE.  Used by oracle/make_golden.py to pin the oracle.
 """
 from __future__ import annotations
 

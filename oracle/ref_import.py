@@ -1,7 +1,6 @@
-"""Import the UNMODIFIED reference classes from /root/reference (build container only).
+"""Import the UNMODIFIED reference classes from a checkout of the reference project ($MAPPERATORINATOR_REFERENCE).
 
-TEST INFRASTRUCTURE. Used only by `oracle/make_golden.py` (fixture generation) and by
-`tests/test_oracle_vs_reference.py` (skipped when /root/reference is absent, i.e. on the GPU box).
+TEST INFRASTRUCTURE. Used only by `oracle/make_golden.py` (fixture generation); the tests read the fixtures.
 Follows the stub recipe of SURVEY.md §8(c): third-party modules that are not installed here
 (hydra, omegaconf, slider, pydub, peft, accelerate, ...) are replaced by MagicMock modules so that
 the reference's own numerics (Mapperatorinator, model_generate, DiT, create_diffusion) import unmodified.
@@ -22,10 +21,6 @@ _STUBS = [
     "accelerate", "accelerate.utils", "accelerate.logging", "matplotlib", "matplotlib.pyplot",
     "nnAudio", "wandb",
 ]
-
-
-def reference_available() -> bool:
-    return os.path.isdir(os.path.join(REFERENCE_ROOT, "osuT5"))
 
 
 def install_stubs() -> None:

@@ -171,26 +171,26 @@ def test_clock_sampler_parses_nvidia_smi_rows():
     assert s["reasons"] == ["hw_thermal_slowdown", "sw_power_cap"]
 
 
-def _trim_cases(layout):
-    """(tokens, trim_lookback, trim_lookahead) cases around both zones; v29 window = 8184 ms, lookback 0.5, lookahead 0.4."""
-    ts, te, circle = layout.time_shift_start, layout.time_shift_end, layout.event_start["circle"]
-    eos, ceos = layout.eos_id, layout.context_eos["map"]
-    lb_end, la_begin = layout.lookback_end(4092.0), layout.lookback_end(4910.4)
-    body = [circle, ts + 500, circle, ts + 520]
-    cases = []
-    for tail in ([], [eos], [ceos], [ceos, eos], [eos, eos, ceos]):
-        for last in (ts, lb_end - 1, lb_end, la_begin - 1, la_begin, te - 1, circle):
-            for tlb in (False, True):
-                for tla in (False, True):
-                    cases.append((body + [circle, last] + tail, tlb, tla))
-    cases += [([], True, True), ([eos], True, True), ([ts + 3], True, True), ([te - 1, eos], False, True)]
-    return cases
+def test_bench_dump_outputs(tmp_path):
+    sys.path.insert(0, ROOT)
+    import bench
+    streams = [[[5, 6, 7], [8, 9]], [[1, 2, 3], [4, 5, 6]]]
+    pos = [torch.full((2, 4), 1.5), torch.full((2, 4), 2.5)]
+    bench.dump_outputs(str(tmp_path / "out"), streams, pos, "_rank1")
+    tok = np.load(tmp_path / "out" / "tokens_rank1.npy")
+    assert tok.dtype == np.float64 and tok.shape == (2, 2, 3)
+    assert tok[0].tolist() == [[5, 6, 7], [8, 9, -1]] and tok[1].tolist() == [[1, 2, 3], [4, 5, 6]]
+    p = np.load(tmp_path / "out" / "positions_rank1.npy")
+    assert p.dtype == np.float32 and p.shape == (2, 2, 4) and p[1].min() == 2.5
+    bench.dump_outputs(str(tmp_path / "dec"), streams, None)
+    assert sorted(os.listdir(tmp_path / "dec")) == ["tokens.npy"]
 
 
 def test_trim_predicted_tokens_properties(layout):
     from mapperatorinator_b200.pipeline import trim_predicted_tokens
+    from oracle import cases
     ts, te = layout.time_shift_start, layout.time_shift_end
-    for toks, tlb, tla in _trim_cases(layout):
+    for toks, tlb, tla in cases.trim_cases(layout):
         for types_first in (True, False):
             out = trim_predicted_tokens(toks, layout, "map", 4092.0, 4910.4, tlb, tla, types_first)
             stripped = list(toks)
@@ -205,31 +205,13 @@ def test_trim_predicted_tokens_properties(layout):
 
 def test_trim_predicted_tokens_matches_reference(layout):
     """The reference's own `Processor.add_predicted_tokens_to_context` (processor.py:1022-1052) run on a stand-in `self` that records what
-    reaches `_decode` — the token-level result this repo's `trim_predicted_tokens` must reproduce."""
-    from oracle import ref_import
-    if not ref_import.reference_available():
-        pytest.skip("/root/reference not present")
-    ref_import.install_stubs()
-    import types
-    from osuT5.osuT5.inference import processor as rp
-    from osuT5.osuT5.tokenizer import ContextType
+    reaches `_decode` (tests/golden/reference_pins.npz) — the token-level result this repo's `trim_predicted_tokens` must reproduce."""
     from mapperatorinator_b200.pipeline import trim_predicted_tokens
-    seen = []
-    fake = types.SimpleNamespace(
-        tokenizer=types.SimpleNamespace(eos_id=layout.eos_id, context_eos={ContextType(k): v for k, v in layout.context_eos.items()}),
-        lookback_time_range=range(layout.time_shift_start, layout.lookback_end(4092.0)),                 # processor.py:85
-        lookahead_time_range=range(layout.lookback_end(4910.4), layout.time_shift_end),                  # processor.py:88
-        types_first=True, eos_time=0.0, lookahead_max_time=4910.4,
-        _decode=lambda toks, frame_time: seen.append(list(toks)) or [], _trim_events_after_time=lambda *a: None)
-    old = rp.update_event_times
-    rp.update_event_times = lambda *a, **k: None
-    try:
-        for types_first in (True, False):
-            fake.types_first = types_first
-            for toks, tlb, tla in _trim_cases(layout):
-                seen.clear()
-                ctx = {"context_type": ContextType("map"), "events": [], "event_times": []}
-                rp.Processor.add_predicted_tokens_to_context(fake, ctx, torch.tensor(toks, dtype=torch.long).tolist(), 1234.0, tlb, tla)
-                assert seen[0] == trim_predicted_tokens(toks, layout, "map", 4092.0, 4910.4, tlb, tla, types_first), (toks, tlb, tla, types_first)
-    finally:
-        rp.update_event_times = old
+    from oracle import cases
+    pins = np.load(os.path.join(ROOT, "tests", "golden", "reference_pins.npz"))
+    off, ref = pins["trim_offsets"], pins["trim_tokens"]
+    runs = [(types_first, c) for types_first in (True, False) for c in cases.trim_cases(layout)]
+    assert len(runs) == len(off) - 1
+    for k, (types_first, (toks, tlb, tla)) in enumerate(runs):
+        want = ref[off[k]:off[k + 1]].tolist()
+        assert want == trim_predicted_tokens(toks, layout, "map", 4092.0, 4910.4, tlb, tla, types_first), (toks, tlb, tla, types_first)

@@ -1,8 +1,8 @@
 """Slider end-point recompute of the diffusion `denoised_fn` (SURVEY §8f N2; diffusion_pipeline.py:203-222, slider_path.py, path_approximator.py).
 
 CPU: the oracle restatement (oracle/slider.py) against tests/golden/slider_reference.npz — end points and path lengths produced by the
-UNMODIFIED reference `SliderPath` on every slider of the reference's toy beatmap plus seeded random control points — and, where
-/root/reference exists, against the reference class directly.
+UNMODIFIED reference `SliderPath` on every slider of the reference's toy beatmap plus seeded random control points — and against
+that class's end points on a second seeded set (tests/golden/reference_pins.npz).
 GPU: the device recompute (csrc/slider.cu, through the C ABI) against the same fixture and against the oracle closure, alone and inside
 the fused 100-step loop.  Tolerance: 1e-3 in normalised coordinates (north_star) = 0.256 px; measured errors are ~1e-3 px.
 """
@@ -38,27 +38,18 @@ def test_oracle_slider_matches_reference_fixture(gold):
     assert worst <= 1e-3, worst                                   # pixels
 
 
-@pytest.mark.reference
 def test_oracle_slider_matches_reference_class():
-    from oracle import ref_import
-    if not ref_import.reference_available():
-        pytest.skip("needs /root/reference")
-    SP = ref_import.reference_slider_path()
-    rng = np.random.default_rng(7)
+    """The oracle against the reference `SliderPath` on 60 seeded sliders per curve type (tests/golden/reference_pins.npz)."""
+    from oracle import cases
+    pins = np.load(os.path.join(GOLDEN, "reference_pins.npz"))
+    sliders = cases.slider_class_cases()
+    assert len(sliders) == len(pins["slider_class_max_length"]) == 240
     worst = 0.0
-    for typ in ("Bezier", "PerfectCurve", "Catmull", "Linear"):
-        for k in range(60):
-            ncp = int(rng.integers(2, 10)) if typ != "PerfectCurve" else int(rng.choice([3, 3, 4, 2]))
-            cps = (rng.random((ncp, 2)) * np.array([512, 384])).astype(np.float32)
-            if ncp >= 4 and k % 4 == 0:
-                j = int(rng.integers(1, ncp - 2)); cps[j + 1] = cps[j]
-            length = float(rng.random() * 500 + 5)
-            sp = SP(typ, cps)
-            ml_ref = float(sp.get_distance())
-            if ml_ref == 0:
-                continue
-            ml, end = so.slider_end_position(typ, cps, length)
-            worst = max(worst, float(np.abs(end - np.asarray(sp.position_at(length / ml_ref), dtype=np.float64)).max()))
+    for (typ, cps, length), ml_ref, end_ref in zip(sliders, pins["slider_class_max_length"], pins["slider_class_end_pos"]):
+        if ml_ref == 0:
+            continue
+        ml, end = so.slider_end_position(typ, cps, length)
+        worst = max(worst, float(np.abs(end - end_ref).max()))
     assert worst <= 1e-3, worst
 
 
